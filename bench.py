@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the Line3D++ matching hot path on B200 (contract: see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scaling weak|strong]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scaling weak|strong] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric: matched line-pairs/sec = (source segment, target segment) pair evaluations per second of the epipolar matching
@@ -19,6 +19,8 @@ One step = all-gather (N>1) + per-segment pre-pass + one fused match/top-k launc
   e2e   : same step through the C ABI with HOST buffers: H2D of this rank's segments from pinned memory, match,
           D2H of the per-row counts and kNN record slots into pinned memory (l3d_match_pairs_host: chunked, the copy
           of a finished chunk overlaps the arithmetic of the next).
+`--dump-outputs DIR` writes what the last timed step computed (see dump_outputs) as DIR/<name>.npy; the inputs are seeded, so two
+builds of the project can be compared output for output.
 `--impl reference` times the reference's CPU/OpenMP matching path (oracle port of matchingCPU, line3D.cc:900-1015;
 line3D.cc itself cannot be compiled in this image) on the host cores, on a bounded sample of the same workload.
 """
@@ -314,6 +316,8 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     launches = (ctx.launch_count() - launches0) / (args.steps + args.warmup)
     pe_local = ctx.match_pair_evals()
+    if args.dump_outputs:
+        dump_outputs(ctx, scene, pairs, args.dump_outputs, f"rank{rank}_" if world > 1 else "")
     e2e_ms = timed(step_e2e, args.steps, max(args.warmup, 1) + 1)   # +1: first call allocates the pinned output buffers
     assert ctx.match_total_rows() == rows_total
     state["total"] = int(state["counts"].sum().item())              # emitted matches, counted from what arrived on the host
@@ -400,6 +404,29 @@ def run_ours(args):
     ctx.close()
     sys.stdout.flush()
     return 0
+
+
+def dump_outputs(ctx, scene, pairs, out_dir, prefix="", nsample=32):
+    """The match result the timed step leaves for its caller (l3d_match_pairs: per source segment of every view pair its match
+    count and kNN records), as float arrays: the number of matches of every view pair, and for a fixed, seeded sample of nsample
+    view pairs the full lists - counts, target segment ids, overlaps and the four depths, with -1 in every field of an empty slot
+    (a match has a positive overlap and positive depths).  About 27 MB for 32 pairs of 3000 x 3000 segments."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts, _ = ctx.match_counts()
+    off = ctx.pair_row_offsets(len(pairs))
+    csum = np.concatenate([[0], np.cumsum(counts, dtype=np.int64)])
+    out = {"matches_per_pair": (csum[off[1:]] - csum[off[:-1]]).astype(np.float64)}
+    sel = np.sort(np.random.default_rng(0).choice(len(pairs), min(nsample, len(pairs)), replace=False))
+    lists = [ctx.pair_matches(int(p), len(scene.segs[pairs[p][0]])) for p in sel]
+    empty = [np.arange(r.shape[1])[None, :] >= c[:, None] for c, r in lists]
+    out["sample_pairs"] = pairs[sel].astype(np.float64)
+    out["sample_counts"] = np.stack([c for c, _ in lists]).astype(np.float32)
+    out["sample_tgt_seg"] = np.stack([np.where(e, -1.0, r["tgt_seg"]) for e, (_, r) in zip(empty, lists)])
+    out["sample_overlap"] = np.stack([np.where(e, -1.0, r["overlap"]).astype(np.float32) for e, (_, r) in zip(empty, lists)])
+    out["sample_depths"] = np.stack([np.where(e[..., None], -1.0, np.stack([r[f] for f in ("d_p1", "d_p2", "d_q1", "d_q2")], -1)).astype(np.float32)
+                                     for e, (_, r) in zip(empty, lists)])
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), a)
 
 
 def nominal_fp32_tflops(clocks):
@@ -538,6 +565,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
     global VIEWS_PER_GPU, SCALING
     SCALING = args.scaling

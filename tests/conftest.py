@@ -14,18 +14,20 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def oracle():
-    """CPU oracle bindings (test infrastructure); builds liboracle.so (and oracle/_ref when /root/reference exists)."""
+    """CPU oracle bindings (test infrastructure); builds liboracle.so.  What the reference itself computes is recorded under
+    tests/golden/."""
     from oracle import pyoracle
-    pyoracle.build(ref=os.path.isdir("/root/reference"))
+    pyoracle.build(ref=False)
     return pyoracle
 
 
 @pytest.fixture(scope="session")
-def ref_nofma(oracle):
-    L = oracle.ref_lib("nofma")
-    if L is None:
-        pytest.skip("oracle/_ref not built (no /root/reference and no prebuilt .so)")
-    return L
+def ref():
+    """outputs of the unmodified reference kernels on a B200, recorded by tests/golden/make_ref_outputs.py: ref(prefix) -> record"""
+    import numpy as np
+    from tests import util
+    z = np.load(os.path.join(ROOT, "tests", "golden", "ref_outputs_gpu_v1.npz"))
+    return lambda prefix: util.load_record(z, prefix)
 
 
 @pytest.fixture(scope="session")

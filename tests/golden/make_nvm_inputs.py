@@ -1,7 +1,7 @@
 """Builds tests/golden/nvm_inputs_v1.npz and tests/golden/line3dpp_ref_fixture_v1.npz from the reference's test data
 (run in the build container, where /root/reference exists and cv2 has an LSD):
 
-    python tests/golden/make_nvm_inputs.py
+    python tests/golden/make_nvm_inputs.py            # python tests/golden/make_nvm_inputs.py --sample: the reader fixture
 
 nvm_inputs_v1.npz: what runLine3Dpp_vsfm hands to Line3D::addImage for testdata/vsfm_result.nvm
   (main_vsfm.cpp:143-310): per camera K (f, w/2, h/2), R (from the quaternion), t = -R C, median world-point depth,
@@ -109,5 +109,18 @@ def main():
     np.savez_compressed(os.path.join(OUT, "line3dpp_ref_fixture_v1.npz"), segs3d=segs, seg_line=seg_line, residuals=res)
 
 
+def sample_nvm(npts=500):
+    """vsfm_result_sample_v1.nvm.gz: testdata/vsfm_result.nvm with every camera line and its PLY trailer verbatim, but only a
+    fixed, seeded sample of npts of its 3D points (lines verbatim, file order kept), for the reader test"""
+    import gzip
+    L = open(os.path.join(REF, "vsfm_result.nvm")).read().split("\n")
+    ncam = int(L[2].split()[0])
+    n = int(L[4 + ncam].split()[0])
+    keep = np.sort(np.random.default_rng(0).choice(n, npts, replace=False))
+    out = L[:4 + ncam] + [str(npts)] + [L[5 + ncam + i] for i in keep] + L[5 + ncam + n:]
+    with gzip.open(os.path.join(OUT, "vsfm_result_sample_v1.nvm.gz"), "wt", compresslevel=9) as f:
+        f.write("\n".join(out))
+
+
 if __name__ == "__main__":
-    sys.exit(main())
+    sys.exit(sample_nvm() if "--sample" in sys.argv else main())

@@ -1,5 +1,6 @@
-"""GPU parity of the matching kernels against the UNMODIFIED reference kernels (oracle/_ref, built with -fmad=false)
-and the CPU oracle.  Everything goes through the C ABI (line3dpp_b200.capi -> libl3d_b200.so)."""
+"""GPU parity of the matching kernels against the UNMODIFIED reference kernels (oracle/_ref, built with -fmad=false; their
+outputs recorded in tests/golden/ref_outputs_gpu_v1.npz by tests/golden/make_ref_outputs.py) and the CPU oracle.  Everything
+goes through the C ABI (line3dpp_b200.capi -> libl3d_b200.so)."""
 import numpy as np
 import pytest
 
@@ -23,60 +24,62 @@ def loaded(gpu_ctx, scene):
 PAIRS = [(0, 1), (0, 4), (2, 3), (5, 1), (7, 6)]
 
 
+def check_lists(counts, recs, r, max_ties=None, what=""):
+    """kNN lists against the recorded reference: same counts, same sets up to exact ties at the k-th place, and (max_ties)
+    at most that many rows whose sets differ at all"""
+    assert np.array_equal(counts, r["counts"]), (what, np.flatnonzero(counts != r["counts"])[:10])
+    assert util.tie_sha(counts, recs) == r["tie_sha"], what
+    if max_ties is not None:
+        assert (util.row_shas(counts, recs) != r["row_sha"]).sum() <= max_ties, what
+    for row in range(len(counts)):
+        ov = recs[row, :counts[row]]["overlap"]
+        assert np.all(ov[:-1] >= ov[1:])
+
+
 @pytest.mark.parametrize("src,tgt", PAIRS)
-def test_dense_bit_exact_vs_reference_kernel(loaded, scene, oracle, ref_nofma, src, tgt):
+def test_dense_bit_exact_vs_reference_kernel(loaded, scene, ref, src, tgt):
     """l3d_match_dense == verbatim K_match_lines (cudawrapper.cu:186-253), every cell, every bit."""
     pi = util.pair_inputs(scene, src, tgt)
-    rdep, rov, _ = oracle.match_dense(ref_nofma.ref_match_dense, pi["ls"], pi["lt"], pi["F"], pi["Rs"], pi["Rt"], pi["Cs"], pi["Ct"], 0.25)
+    r = ref(f"dense/{src}_{tgt}")
     dep, ov = loaded.match_dense(src, tgt, pi["F"], 0.25, len(pi["ls"]), len(pi["lt"]))
-    assert np.array_equal(util.bits(ov), util.bits(rov))
-    assert np.array_equal(util.bits(dep), util.bits(rdep))
+    assert util.sha(util.bits(ov)) == r["ov_sha"]
+    assert util.sha(util.bits(dep)) == r["dep_sha"]
     # the conservative pre-filter must never change a result
     dep2, ov2 = loaded.match_dense(src, tgt, pi["F"], 0.25, len(pi["ls"]), len(pi["lt"]), nofilter=True)
-    assert np.array_equal(util.bits(ov2), util.bits(rov)) and np.array_equal(util.bits(dep2), util.bits(rdep))
-    assert (rov > 0.25).sum() > 100   # the case is not vacuous
+    assert util.sha(util.bits(ov2)) == r["ov_sha"] and util.sha(util.bits(dep2)) == r["dep_sha"]
+    assert r["nsel"] > 100   # the case is not vacuous
 
 
 @pytest.mark.parametrize("src,tgt", PAIRS[:3])
-def test_dense_cpu_oracle_matches_reference(scene, oracle, ref_nofma, src, tgt):
-    """pins the CPU restatement: overlap bit-exact, depths to 1e-5 relative (host rsqrt differs from MUFU.RSQ)."""
+def test_dense_cpu_oracle_matches_reference(scene, oracle, ref, src, tgt):
+    """pins the CPU restatement: overlap bit-exact, depths to 1e-5 relative (host rsqrt differs from MUFU.RSQ) on a seeded
+    sample of the cells above the threshold."""
     pi = util.pair_inputs(scene, src, tgt)
-    rdep, rov, _ = oracle.match_dense(ref_nofma.ref_match_dense, pi["ls"], pi["lt"], pi["F"], pi["Rs"], pi["Rt"], pi["Cs"], pi["Ct"], 0.25)
+    r = ref(f"dense/{src}_{tgt}")
     odep, oov, _ = oracle.match_dense(oracle.lib().orc_match_dense_f32, pi["ls"], pi["lt"], pi["F"], pi["Rs"], pi["Rt"], pi["Cs"], pi["Ct"], 0.25)
-    assert np.array_equal(util.bits(oov), util.bits(rov))
-    sel = rov > 0.25
-    rel = np.abs(odep[sel] - rdep[sel]) / np.maximum(np.abs(rdep[sel]), 1e-3)
+    assert util.sha(util.bits(oov)) == r["ov_sha"]
+    sel = np.flatnonzero(oov.reshape(-1) > 0.25)
+    assert len(sel) == r["nsel"] and np.array_equal(sel[util.pick(len(sel))], r["cells"])
+    odep, rdep = odep.reshape(-1, 4)[r["cells"]], r["dep"]
+    rel = np.abs(odep - rdep) / np.maximum(np.abs(rdep), 1e-3)
     assert np.median(rel) < 1e-6 and np.quantile(rel, 0.999) < 1e-2     # ill-conditioned depths (n.ray ~ 0) amplify the rsqrt difference
-    assert np.array_equal(np.sign(odep[sel]), np.sign(rdep[sel])) or (np.sign(odep[sel]) != np.sign(rdep[sel])).mean() < 1e-5
+    assert np.array_equal(np.sign(odep), np.sign(rdep)) or (np.sign(odep) != np.sign(rdep)).mean() < 1e-5
 
 
-def test_topk_vs_reference_wrapper(loaded, scene, oracle, ref_nofma):
+def test_topk_vs_reference_wrapper(loaded, scene, ref):
     """l3d_match_pairs == verbatim match_lines_GPU (kernel + D2H + host priority queue, cudawrapper.cu:549-658):
-    same match set per source segment, bit-exact payload.  Order inside a row: overlap descending."""
+    same match set per source segment, bit-exact payload.  Order inside a row: overlap descending.  The only acceptable
+    difference is a tie in overlap at the k-th place (std::priority_queue order is unspecified), in at most 2 rows."""
     pairs = np.array(PAIRS, np.int32)
     loaded.match_pairs(pairs, util.pair_F(scene, pairs), 0.25, 10)
     for p, (src, tgt) in enumerate(PAIRS):
-        pi = util.pair_inputs(scene, src, tgt)
-        rcounts, rout, rtotal, _ = oracle.match_lines(ref_nofma.ref_match_lines, pi["ls"], pi["lt"], pi["F"], pi["Rs"], pi["Rt"], pi["Cs"], pi["Ct"], src, tgt, 0.25, 10)
-        counts, recs = loaded.pair_matches(p, len(pi["ls"]))
-        assert np.array_equal(counts, rcounts)
-        assert rtotal == counts.sum() and rtotal > 1000
-        mine = util.rows_as_sets(counts, recs)
-        ref = util.rows_as_sets(rcounts, rout)
-        nties = 0
-        for r in range(len(counts)):
-            if mine[r] != ref[r]:
-                # only acceptable difference: a tie in overlap at the k-th place (std::priority_queue order is unspecified)
-                kth = min(e[1] for e in ref[r])
-                assert {e for e in mine[r] if e[1] != kth} == {e for e in ref[r] if e[1] != kth}, (src, tgt, r)
-                nties += 1
-            ov = recs[r, :counts[r]]["overlap"]
-            assert np.all(ov[:-1] >= ov[1:])
-        assert nties <= 2
+        counts, recs = loaded.pair_matches(p, len(scene.segs[src]))
+        check_lists(counts, recs, ref(f"topk/{src}_{tgt}"), max_ties=2, what=(src, tgt))
+        assert counts.sum() > 1000
 
 
 @pytest.mark.parametrize("f64", [False, True])
-def test_keep_all_matches(loaded, scene, oracle, ref_nofma, f64):
+def test_keep_all_matches(loaded, scene, oracle, ref, f64):
     """kNN <= 0: every cell with overlap > epi and positive depths is kept, in ascending target order
     (cudawrapper.cu:628-636 / line3D.cc:988-996) -- against the verbatim wrapper (float) and the oracle's matchingCPU (double)"""
     pairs = np.array(PAIRS[:3], np.int32)
@@ -94,12 +97,12 @@ def test_keep_all_matches(loaded, scene, oracle, ref_nofma, f64):
             RtKinv, C = synth.camera_blocks(scene)
             rcounts, rout, rtotal, _ = oracle.match_lines(oracle.lib().orc_match_lines_f64, pi["ls"], pi["lt"], Fd[p], RtKinv[src].reshape(9),
                                                           RtKinv[tgt].reshape(9), C[src], C[tgt], src, tgt, 0.25, 0, f64=True)
-        else:
-            rcounts, rout, rtotal, _ = oracle.match_lines(ref_nofma.ref_match_lines, pi["ls"], pi["lt"], pi["F"], pi["Rs"], pi["Rt"], pi["Cs"],
-                                                          pi["Ct"], src, tgt, 0.25, 0)
         counts, recs = loaded.pair_matches(p, len(pi["ls"]))
-        assert np.array_equal(counts, rcounts) and rtotal == counts.sum()
         biggest = max(biggest, int(counts.max()))
+        if not f64:
+            assert util.list_sha(counts, recs) == ref(f"keep_all/{src}_{tgt}")["list_sha"], (src, tgt)    # same members, same ORDER, bit-exact payload
+            continue
+        assert np.array_equal(counts, rcounts) and rtotal == counts.sum()
         for r in range(len(counts)):
             a, b = recs[r, :counts[r]], rout[r, :counts[r]]
             for f in ("tgt_seg", "overlap", "d_p1", "d_p2", "d_q1", "d_q2"):
@@ -107,22 +110,18 @@ def test_keep_all_matches(loaded, scene, oracle, ref_nofma, f64):
     assert biggest <= stride
 
 
-def test_keep_all_pipeline_vs_reference_kernels(oracle, ref_nofma):
+def test_keep_all_pipeline_vs_reference_kernels(ref):
     """matchImages(kNN = -1) end to end: scored matches bit-identical to the reference kernels behind the oracle host logic"""
     from line3dpp_b200 import line3d
     sc = synth.make_scene(6, 250, 13, "ring2")
     L = line3d.Line3D(neighbors_by_worldpoints=False)
     L.add_scene(sc); L.match_images(knn=-1)
-    P = oracle.OraclePipeline(False, True, backend=ref_nofma)
-    P.add_scene(sc); P.match_images(knn=-1)
-    n = 0
-    for cam in sc.cam_ids:
-        g, o = L.view_matches(cam, False), P.scored(cam)
-        assert g.tobytes() == o.tobytes(), f"view {cam}"
-        n += len(g)
-    assert n > 3000
-    L.reconstruct_3d_lines(3, False); assert P.reconstruct(3, False) == 0
-    assert L.stats()["lines3D"] == P.num_lines() > 20
+    r = ref("keep_all_pipeline")
+    mine = util.stage_record(scored=[L.view_matches(cam, False) for cam in sc.cam_ids])
+    assert np.array_equal(mine["scored_n"], r["scored_n"]) and mine["scored_sha"] == r["scored_sha"]
+    assert r["scored_n"].sum() > 3000
+    L.reconstruct_3d_lines(3, False)
+    assert L.stats()["lines3D"] == r["num_lines"] > 20
     L.close()
 
 
@@ -300,7 +299,7 @@ def test_capi_error_behaviour(gpu_ctx):
     fresh.close()
 
 
-def test_knn_above_32_vs_reference_wrapper(loaded, scene, oracle, ref_nofma):
+def test_knn_above_32_vs_reference_wrapper(loaded, scene, ref):
     """kNN > 32 (beyond the fused kernel's per-row key list; the reference accepts any kNN, cudawrapper.cu:637-645): the keep-all
     passes + per-row cut must give the reference wrapper's matches, in its pop order (overlap descending)."""
     knn = 40
@@ -309,18 +308,10 @@ def test_knn_above_32_vs_reference_wrapper(loaded, scene, oracle, ref_nofma):
     loaded.match_pairs(pairs, util.pair_F(scene, pairs), 0.05, knn)       # low threshold: rows longer than 32 exist
     nlong = 0
     for p, (src, tgt) in enumerate(PAIRS[:2]):
-        pi = util.pair_inputs(scene, src, tgt)
-        rcounts, rout, rtotal, _ = oracle.match_lines(ref_nofma.ref_match_lines, pi["ls"], pi["lt"], pi["F"], pi["Rs"], pi["Rt"], pi["Cs"], pi["Ct"], src, tgt, 0.05, knn)
-        counts, recs = loaded.pair_matches(p, len(pi["ls"]))
-        assert np.array_equal(counts, rcounts) and counts.max() <= knn
+        counts, recs = loaded.pair_matches(p, len(scene.segs[src]))
+        check_lists(counts, recs, ref(f"knn40/{src}_{tgt}"), what=(src, tgt))
+        assert counts.max() <= knn
         nlong += int((counts > 32).sum())
-        mine, ref = util.rows_as_sets(counts, recs), util.rows_as_sets(rcounts, rout)
-        for r in range(len(counts)):
-            if mine[r] != ref[r]:
-                kth = min(e[1] for e in ref[r])
-                assert {e for e in mine[r] if e[1] != kth} == {e for e in ref[r] if e[1] != kth}, (src, tgt, r)
-            ov = recs[r, :counts[r]]["overlap"]
-            assert np.all(ov[:-1] >= ov[1:])
     assert nlong > 0, "the test scene must have rows with more than 32 matches"
 
 
@@ -345,39 +336,19 @@ def test_dense_batch_equals_single_launches(loaded, scene):
 
 
 @pytest.mark.parametrize("kind", ["sideways", "forward", "edge", "rolled"])
-def test_level1_prefilter_never_drops(gpu_ctx, oracle, ref_nofma, kind):
+def test_level1_prefilter_never_drops(gpu_ctx, ref, kind):
     """the pencil-parameter pre-filter (k_pair_arcs, l3d_device.cuh) with the epipole at infinity, inside the image, near its border
     and with a rolled camera: same matches as the unmodified reference kernel + host kNN pass (which evaluate every cell), both
     directions; horizontal / vertical / tiny segments and segments through the epipole added on purpose"""
-    sc = util.two_view_scene(kind, 1500, 31)
-    rng = np.random.default_rng(5)
-    for v in range(2):
-        s = sc.segs[v]
-        extra = []
-        for _ in range(60):           # axis-parallel segments (parallel to the epipolar lines in the sideways case) and 1-2 px stubs
-            x, y, l = rng.uniform(50, 2900), rng.uniform(50, 2200), rng.uniform(20, 400)
-            extra += [(x, y, min(x + l, 3060), y), (x, y, x, min(y + l, 2290)), (x, y, x + 1.5, y + 0.5)]
-        cx, cy = 1647.1, 1068.7                   # the epipole of the "forward" pair (0, 1): segments through / next to it
-        for a in np.linspace(0, np.pi, 24, endpoint=False):
-            extra += [(cx - 200 * np.cos(a), cy - 200 * np.sin(a), cx + 300 * np.cos(a), cy + 300 * np.sin(a)),
-                      (cx + 3 * np.cos(a), cy + 3 * np.sin(a), cx + 150 * np.cos(a), cy + 150 * np.sin(a))]
-        sc.segs[v] = np.ascontiguousarray(np.concatenate([s, np.array(extra, np.float32)]))
+    sc = util.level1_scene(kind)
     gpu_ctx.set_views(util.scene_descs(sc), sc.segs)
     pairs = np.array([(0, 1), (1, 0)], np.int32)
     for epi, knn in ((0.25, 10), (0.05, 32)):
         gpu_ctx.match_pairs(pairs, util.pair_F(sc, pairs), epi, knn)
         tot = 0
         for p, (s, t) in enumerate(pairs):
-            pi = util.pair_inputs(sc, s, t)
-            oc, oo, _, _ = oracle.match_lines(ref_nofma.ref_match_lines, pi["ls"], pi["lt"], pi["F"], pi["Rs"], pi["Rt"], pi["Cs"], pi["Ct"], s, t, epi, knn)
-            counts, recs = gpu_ctx.pair_matches(p, len(pi["ls"]))
-            assert np.array_equal(counts, oc), (kind, s, t, epi, np.flatnonzero(counts != oc)[:10])
-            f = ("tgt_seg", "overlap", "d_p1", "d_p2", "d_q1", "d_q2")
-            ours, theirs = util.rows_as_sets(counts, recs, f), util.rows_as_sets(oc, oo, f)
-            for row, (a, b) in enumerate(zip(ours, theirs)):
-                if a != b:      # only an exact tie in the k-th place may differ (DESIGN section 2: the reference pops an unordered heap)
-                    assert sorted(x[1] for x in a) == sorted(x[1] for x in b), (kind, s, t, epi, row)
-                    kth = min(x[1] for x in a)
-                    assert all(x[1] == kth for x in set(a) ^ set(b)), (kind, s, t, epi, row)
+            counts, recs = gpu_ctx.pair_matches(p, len(sc.segs[s]))
+            # only an exact tie in the k-th place may differ (DESIGN section 2: the reference pops an unordered heap)
+            check_lists(counts, recs, ref(f"level1_{kind}_{epi}_{knn}/{s}_{t}"), what=(kind, s, t, epi))
             tot += int(counts.sum())
         assert tot > 1000          # not vacuous

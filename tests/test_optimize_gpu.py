@@ -1,12 +1,14 @@
 """GPU parity of the line bundling (SURVEY.md §8f-4): l3d_optimize_lines against
   * the reference's OWN Ceres run: testdata/Line3D++_ref before / after result files (tests/golden/make_opt_fixture.py),
   * the oracle restatement of the same trust-region minimiser (same iterates, so agreement to rounding),
-and the use_CERES flag of reconstruct3Dlines through the L3DPP::Line3D mirror against the oracle pipeline."""
+and the use_CERES flag of reconstruct3Dlines through the L3DPP::Line3D mirror against the oracle pipeline driven by the
+reference kernels (recorded in tests/golden/ref_outputs_gpu_v1.npz by tests/golden/make_ref_outputs.py)."""
 import numpy as np
 import pytest
 
 from line3dpp_b200 import synth, line3d
 from tests import nvm_util as nu
+from tests import util
 
 pytestmark = pytest.mark.gpu
 
@@ -63,7 +65,7 @@ def test_subsets_ragged_and_degenerate_lines(gpu_ctx, oracle, pairs):
 
 
 @pytest.mark.parametrize("diffusion", [False, True])
-def test_use_ceres_through_line3d_vs_oracle_pipeline(oracle, ref_nofma, diffusion):
+def test_use_ceres_through_line3d_vs_oracle_pipeline(ref, diffusion):
     sc = synth.make_scene(12, 500, 96, "ring3", noise_px=1.0)
     L = line3d.Line3D(neighbors_by_worldpoints=False, use_gpu=True)
     L.add_scene(sc)
@@ -72,21 +74,15 @@ def test_use_ceres_through_line3d_vs_oracle_pipeline(oracle, ref_nofma, diffusio
     plain = L.segments3d()
     L.reconstruct_3d_lines(3, diffusion, -1.0, True, 250)
     st = L.stats()
-    P = oracle.OraclePipeline(False, True, backend=ref_nofma)
-    P.add_scene(sc)
-    P.match_images()
-    assert P.reconstruct(3, diffusion, -1.0, True, 250) == 0
-    sm = P.opt_summary()
+    r = ref(f"ceres/{diffusion}")
+    sm = r["opt_summary"]
     assert st["opt_iterations"] == sm[0] and st["opt_iterations"] > 3
     np.testing.assert_allclose([st["opt_cost_before"], st["opt_cost_after"]], sm[1:3], rtol=1e-7)
     assert st["opt_cost_after"] < st["opt_cost_before"]
-    assert st["lines3D"] == P.num_lines()
-    mr, orr = L.residuals(), P.residuals()
-    assert np.array_equal(mr["line"], orr["line"]) and np.array_equal(mr["cam"], orr["cam"]) and np.array_equal(mr["seg"], orr["seg"])
-    ms, os_ = L.segments3d(), P.segments3d()
-    a = np.sort(np.stack([ms["p1"], ms["p2"]], 1), axis=1)
-    b = np.sort(np.stack([os_["p1"], os_["p2"]], 1), axis=1)
-    np.testing.assert_allclose(a, b, atol=1e-6)     # TOLERANCE on 3D endpoint positions: 1e-6 scene units
+    ms = L.segments3d()
+    mine = util.stage_record(num_lines=st["lines3D"], residuals=L.residuals(), segments=ms)
+    keys = ("num_lines", "res_line_sha", "res_camseg_sha", "seg_n", "seg_pts_smp")
+    util.check_record(mine, {k: r[k] for k in keys}, {"seg_pts_smp": dict(atol=1e-6)})     # TOLERANCE on 3D endpoint positions: 1e-6 scene units
 
     def gt(s):
         g = sc.lines3d; o = g[:, :3]; d = g[:, 3:] - o; d = d / np.linalg.norm(d, axis=1, keepdims=True)
@@ -99,7 +95,7 @@ def test_use_ceres_through_line3d_vs_oracle_pipeline(oracle, ref_nofma, diffusio
     L.close()
 
 
-def test_nvm_with_bundling_vs_optimized_fixture(oracle, ref_nofma):
+def test_nvm_with_bundling_vs_optimized_fixture(ref):
     """testdata/vsfm_result.nvm with use_CERES on the B200 against the reference's OPTIMIZED result (statistical: the 2D
     segments of the fixture run are not reproducible, SURVEY.md §4) and against the oracle pipeline (1e-6)"""
     inp = nu.load_inputs()
@@ -108,15 +104,11 @@ def test_nvm_with_bundling_vs_optimized_fixture(oracle, ref_nofma):
     nu.add_all(L.add_image, inp)
     L.match_images()
     L.reconstruct_3d_lines(3, False, -1.0, True, 250)
-    P = oracle.OraclePipeline(True, 1, backend=ref_nofma)
-    nu.add_all(P.add_view, inp)
-    assert P.match_images() == 0 and P.reconstruct(3, False, -1.0, True, 250) == 0
+    r = ref("ceres/nvm")
     st = L.stats()
-    assert st["lines3D"] == P.num_lines() and st["opt_iterations"] == P.opt_summary()[0]
-    ms, os_ = L.segments3d(), P.segments3d()
-    a = np.sort(np.stack([ms["p1"], ms["p2"]], 1), axis=1)
-    b = np.sort(np.stack([os_["p1"], os_["p2"]], 1), axis=1)
-    np.testing.assert_allclose(a, b, atol=1e-6)
+    assert st["lines3D"] == r["num_lines"] and st["opt_iterations"] == r["opt_summary"][0]
+    ms = L.segments3d()
+    util.check_record(util.stage_record(segments=ms), {k: r[k] for k in ("seg_n", "seg_pts_smp")}, {"seg_pts_smp": dict(atol=1e-6)})
     assert abs(st["lines3D"] - len(after)) <= 0.03 * len(after)
     mine = np.concatenate([ms["p1"], ms["p2"]], 1)
     depth = float(np.median(inp["median_depth"]))

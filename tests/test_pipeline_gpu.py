@@ -6,6 +6,7 @@ The oracle's host logic (oracle/l3d_oracle.cc) is driven twice:
     reference GPU path except for line3D.cc's host glue; the product must agree index-exactly and bit-exactly on
     overlaps / depths / scores;
   * with its CPU emulation, to show the same at libm tolerance.
+What the reference kernels computed is recorded in tests/golden/ref_outputs_gpu_v1.npz (tests/golden/make_ref_outputs.py).
 """
 import numpy as np
 import pytest
@@ -31,11 +32,8 @@ def product(scene):
 
 
 @pytest.fixture(scope="module")
-def oracle_ref(scene, oracle, ref_nofma):
-    P = oracle.OraclePipeline(False, True, backend=ref_nofma)
-    P.add_scene(scene)
-    assert P.match_images() == 0
-    return P
+def product_match(product, scene):
+    return util.product_record(product, scene.cam_ids, None, recon=False)
 
 
 @pytest.fixture(scope="module")
@@ -46,45 +44,25 @@ def oracle_cpu(scene, oracle):
     return P
 
 
-def _same_matches(a, b, exact_scores):
-    assert len(a) == len(b)
-    for f in ("src_cam", "src_seg", "tgt_cam", "tgt_seg"):
-        assert np.array_equal(a[f], b[f]), f
-    for f in ("overlap", "d_p1", "d_p2", "d_q1", "d_q2"):
-        assert np.array_equal(util.bits(a[f]), util.bits(b[f])), f
-    if exact_scores:
-        assert np.array_equal(util.bits(a["score3D"]), util.bits(b["score3D"]))
-    else:
-        np.testing.assert_allclose(a["score3D"], b["score3D"], rtol=2e-5, atol=2e-6)
+def test_view_pairs_and_regularisers(product_match, ref):
+    r = ref("pipeline/match")
+    assert product_match["pairs_sha"] == r["pairs_sha"]
+    assert np.array_equal(product_match["view_info"], r["view_info"])
 
 
-def test_view_pairs_and_regularisers(product, oracle_ref, scene):
-    assert np.array_equal(product.pairs(), oracle_ref.pairs())
-    for cam in scene.cam_ids:
-        k1, md1 = product.view_info(cam)
-        k2, md2 = oracle_ref.view_info(cam)
-        assert k1 == k2 and md1 == md2, cam
-
-
-def test_scored_matches_bit_exact_vs_reference_kernels(product, oracle_ref, scene):
+def test_scored_matches_bit_exact_vs_reference_kernels(product_match, ref):
     """all matches of every view right after scoring: order, ids, overlap, depths AND score3D bit-identical"""
-    total = 0
-    for cam in scene.cam_ids:
-        mine = product.view_matches(cam, kept_only=False)
-        ref = oracle_ref.scored(cam)
-        _same_matches(mine, ref, exact_scores=True)
-        total += len(mine)
-    assert total > 20000
+    r = ref("pipeline/match")
+    assert np.array_equal(product_match["scored_n"], r["scored_n"]) and product_match["scored_sha"] == r["scored_sha"]
+    assert r["scored_n"].sum() > 20000
 
 
-def test_kept_matches_and_estimates_vs_reference_kernels(product, oracle_ref, scene):
-    for cam in scene.cam_ids:
-        _same_matches(product.view_matches(cam, kept_only=True), oracle_ref.matches(cam), exact_scores=True)
-    best, p = product.estimates()
-    obest, op = oracle_ref.estimates()
-    _same_matches(best, obest, exact_scores=True)
-    np.testing.assert_allclose(p, op, rtol=0, atol=1e-12)
-    assert len(best) > 2000
+def test_kept_matches_and_estimates_vs_reference_kernels(product_match, ref):
+    r = ref("pipeline/match")
+    assert np.array_equal(product_match["kept_n"], r["kept_n"]) and product_match["kept_sha"] == r["kept_sha"]
+    assert product_match["est_n"] == r["est_n"] and product_match["est_sha"] == r["est_sha"]
+    np.testing.assert_allclose(product_match["est_p_smp"], r["est_p_smp"], rtol=0, atol=1e-12)
+    assert r["est_n"] > 2000
 
 
 def test_scored_matches_vs_cpu_oracle(product, oracle_cpu, scene):
@@ -106,74 +84,44 @@ def test_scored_matches_vs_cpu_oracle(product, oracle_cpu, scene):
     assert nbad <= 3 and ntot > 10000 and noff / ntot < 0.01
 
 
+# affinity weights: host libm vs libdevice; TOLERANCE on 3D endpoint positions: 1e-6 scene units
+RECON_TOL = {"affraw_w_smp": dict(rtol=1e-5), "aff_w_smp": dict(rtol=1e-4, atol=1e-12), "seg_pts_smp": dict(atol=1e-6)}
+
+
 @pytest.mark.parametrize("diffusion", [False, True])
-def test_reconstruction_vs_reference_kernels(scene, oracle, ref_nofma, diffusion):
+def test_reconstruction_vs_reference_kernels(scene, ref, diffusion):
+    """affinity matrix before diffusion: same local ids, same edges in the same order, weights to libm tolerance; the matrix handed
+    to the clustering (after diffusion if enabled); 3D lines (end points compared unordered: their order depends on the sign of
+    the principal axis)"""
     L = line3d.Line3D(neighbors_by_worldpoints=False, use_gpu=True)
     L.add_scene(scene)
     L.match_images()
     L.reconstruct_3d_lines(3, diffusion)
-    P = oracle.OraclePipeline(False, True, backend=ref_nofma)
-    P.add_scene(scene)
-    P.match_images()
-    assert P.reconstruct(3, diffusion) == 0
-    # affinity matrix before diffusion: same local ids, same edges in the same order, weights to libm tolerance
-    assert np.array_equal(L.local2global(), P.local2global())
-    ei, ej, ew = L.affinity(raw=True)
-    oi, oj, ow = P.affinity_raw()
-    assert np.array_equal(ei, oi) and np.array_equal(ej, oj)
-    np.testing.assert_allclose(ew, ow, rtol=1e-5)
-    # matrix handed to the clustering (after diffusion if enabled)
-    ei, ej, ew = L.affinity(raw=False)
-    oi, oj, ow = P.affinity()
-    assert np.array_equal(ei, oi) and np.array_equal(ej, oj)
-    np.testing.assert_allclose(ew, ow, rtol=1e-4, atol=1e-12)
-    # 3D lines
-    st = L.stats()
-    assert st["lines3D"] == P.num_lines() and st["lines3D"] > 100
-    mr, orr = L.residuals(), P.residuals()
-    assert np.array_equal(mr["line"], orr["line"]) and np.array_equal(mr["cam"], orr["cam"]) and np.array_equal(mr["seg"], orr["seg"])
-    ms, os_ = L.segments3d(), P.segments3d()
-    assert np.array_equal(ms["line"], os_["line"])
-    # endpoint order of a segment depends on the sign of the principal axis: compare unordered
-    a = np.sort(np.stack([ms["p1"], ms["p2"]], 1), axis=1)
-    b = np.sort(np.stack([os_["p1"], os_["p2"]], 1), axis=1)
-    np.testing.assert_allclose(a, b, atol=1e-6)     # TOLERANCE on 3D endpoint positions: 1e-6 scene units
+    r = ref(f"pipeline/recon_{diffusion}")
+    util.check_record(util.product_record(L, scene.cam_ids, None, matching=False), r, RECON_TOL)
+    assert r["num_lines"] > 100
     L.close()
 
 
-def test_rdd_bit_exact_vs_reference(gpu_ctx, oracle, ref_nofma):
+def test_rdd_bit_exact_vs_reference(gpu_ctx, oracle, ref):
     """l3d_rdd == verbatim SparseMatrix + replicator_dynamics_diffusion_GPU on a random symmetric affinity graph"""
     import ctypes as C
-    rng = np.random.default_rng(3)
-    n = 3000
-    a = rng.integers(0, n, 40000); b = rng.integers(0, n, 40000)
-    keep = a != b
-    a, b = a[keep], b[keep]
-    key = np.minimum(a, b) * n + np.maximum(a, b)
-    _, idx = np.unique(key, return_index=True)
-    a, b = a[np.sort(idx)], b[np.sort(idx)]
-    # every node needs at least one edge (the reference kernel reads start index -1 otherwise)
-    missing = np.setdiff1d(np.arange(n), np.concatenate([a, b]))
-    a = np.concatenate([a, missing]); b = np.concatenate([b, (missing + 1) % n])
-    w = rng.uniform(0.5, 1.0, len(a)).astype(np.float32)
-    ei = np.stack([a, b], 1).reshape(-1).astype(np.int32)       # (i,j),(j,i) consecutive like A_
-    ej = np.stack([b, a], 1).reshape(-1).astype(np.int32)
-    ew = np.repeat(w, 2)
-    ri, rj, rw, _ = oracle.rdd(ref_nofma.ref_rdd, ei, ej, ew, n)
+    ei, ej, ew, n = util.rdd_graph()
+    r = ref("rdd")
     L = gpu_ctx.L
     oi, oj, ow = np.zeros_like(ei), np.zeros_like(ej), np.zeros_like(ew)
     ms = C.c_float(0)
     p = lambda x: x.ctypes.data_as(C.c_void_p)
     rc = L.l3d_rdd(gpu_ctx.h, n, C.c_longlong(len(ei)), p(ei), p(ej), p(ew), 10, p(oi), p(oj), p(ow), C.byref(ms))
     assert rc == 0
-    assert np.array_equal(oi, ri) and np.array_equal(oj, rj)
-    assert np.array_equal(util.bits(ow), util.bits(rw))
+    assert util.sha(oi.astype(np.int64), oj.astype(np.int64)) == r["idx_sha"]
+    assert util.sha(util.bits(ow)) == r["w_sha"]
     ci, cj, cw, _ = oracle.rdd(oracle.lib().orc_rdd_f32, ei, ej, ew, n)
-    assert np.array_equal(ci, ri) and np.array_equal(util.bits(cw), util.bits(rw))     # pins the CPU restatement too
+    assert util.sha(ci.astype(np.int64), cj.astype(np.int64)) == r["idx_sha"] and util.sha(util.bits(cw)) == r["w_sha"]     # pins the CPU restatement too
 
 
 # ---------------------------------------------------------------------------------------------- BASELINE configs[1]: vsfm_result.nvm on 1 x B200
-def test_nvm_b200_vs_reference_kernels_and_fixture(oracle, ref_nofma):
+def test_nvm_b200_vs_reference_kernels_and_fixture(ref):
     """testdata/vsfm_result.nvm through L3DPP::Line3D on the B200 (neighbours from world points, default parameters):
     index-exact against the oracle host logic driving the UNMODIFIED reference kernels, 3D endpoints within 1e-6 scene
     units, and statistically equal to the reference's own result fixture testdata/Line3D++_ref."""
@@ -184,21 +132,12 @@ def test_nvm_b200_vs_reference_kernels_and_fixture(oracle, ref_nofma):
     nu.add_all(L.add_image, inp)
     L.match_images()
     L.reconstruct_3d_lines(3, False)
-    P = oracle.OraclePipeline(True, 1, backend=ref_nofma)
-    nu.add_all(P.add_view, inp)
-    assert P.match_images() == 0 and P.reconstruct(3, False) == 0
-    assert np.array_equal(L.pairs(), P.pairs())
-    for cam in range(inp["V"]):
-        _same_matches(L.view_matches(cam, kept_only=True), P.matches(cam), exact_scores=True)
-    assert np.array_equal(L.local2global(), P.local2global())
+    r = ref("pipeline/nvm")
+    mine = util.product_record(L, range(inp["V"]), None)
+    keys = ("pairs_sha", "kept_n", "kept_sha", "l2g_sha", "num_lines", "res_camseg_sha", "seg_n", "seg_pts_smp")
+    util.check_record(mine, {k: r[k] for k in keys}, {"seg_pts_smp": dict(atol=1e-6)})
     st = L.stats()
-    assert st["lines3D"] == P.num_lines()
-    mr, orr = L.residuals(), P.residuals()
-    assert np.array_equal(mr["cam"], orr["cam"]) and np.array_equal(mr["seg"], orr["seg"])
-    ms, os_ = L.segments3d(), P.segments3d()
-    a = np.sort(np.stack([ms["p1"], ms["p2"]], 1), axis=1)
-    b = np.sort(np.stack([os_["p1"], os_["p2"]], 1), axis=1)
-    np.testing.assert_allclose(a, b, atol=1e-6)
+    ms = L.segments3d()
     # statistical comparison with the reference's own output
     n_ref = len(set(fl.tolist()))
     assert abs(st["lines3D"] - n_ref) <= 0.03 * n_ref, (st["lines3D"], n_ref)

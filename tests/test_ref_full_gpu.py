@@ -1,7 +1,8 @@
 """The product (L3DPP::Line3D mirror on the B200) against the reference's WHOLE pipeline, UNMODIFIED: line3D.cc + view.cc +
 cudawrapper.cu + sparsematrix.cc + clustering.cc compiled verbatim (oracle/_ref/libl3dref_full_gpu.so, nvcc -fmad=false, Eigen /
 OpenCV / Boost replaced by the stand-ins of oracle/ref_shim) and run live on the same GPU through its own public calls
-addImage / matchImages / reconstruct3Dlines.  No restated host logic is involved in these comparisons.
+addImage / matchImages / reconstruct3Dlines.  No restated host logic is involved in these comparisons; what the reference
+computed is recorded in tests/golden/ref_outputs_gpu_v1.npz (tests/golden/make_ref_outputs.py).
 
 REF_GPU semantics: match ids, overlaps, depths and score3D bit-identical, list order identical, local ids / affinity edges
 index-identical (weights: host libm vs libdevice, 1e-5 relative), 3D end points within 1e-6 scene units.
@@ -14,79 +15,29 @@ import pytest
 
 from line3dpp_b200 import line3d, synth
 from tests import util
-from tests.test_ref_full_cpu import IDS, GEO, check_against_nvm_golden, check_reconstruction_against_nvm_golden
+from tests.test_ref_full_cpu import digest_matches, G
 
 pytestmark = pytest.mark.gpu
 
-
-@pytest.fixture(scope="module")
-def ref_gpu(oracle):
-    if oracle.ref_full_lib("gpu") is None:
-        pytest.skip("oracle/_ref/libl3dref_full_gpu.so not built")
-    return oracle
-
-
-def same_matches_exact(a, b, what):
-    assert len(a) == len(b), (what, len(a), len(b))
-    for f in IDS:
-        assert np.array_equal(a[f], b[f]), (what, f)
-    for f in GEO + ("score3D",):
-        assert np.array_equal(util.bits(a[f]), util.bits(b[f])), (what, f)
-
-
-def compare_all_stages(L, R, cams, nsegs, diffusion, collin):
-    assert np.array_equal(L.pairs(), R.pairs())
-    total = 0
-    for cam in cams:
-        same_matches_exact(L.view_matches(cam, kept_only=False), R.scored(cam), f"scored {cam}")
-        same_matches_exact(L.view_matches(cam, kept_only=True), R.matches(cam), f"kept {cam}")
-        assert L.view_info(cam) == R.view_info(cam), cam
-        total += len(R.scored(cam))
-    best, p = L.estimates()
-    rbest, rp = R.estimates()
-    same_matches_exact(best, rbest, "estimates")
-    np.testing.assert_allclose(p, rp, rtol=0, atol=1e-12)
-    if collin > 0:
-        for vi, cam in enumerate(cams):
-            a, b = L.ctx_collinear(vi, nsegs[vi]), R.collinear(cam, nsegs[vi])
-            assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), cam
-    assert np.array_equal(L.local2global(), R.local2global())
-    ei, ej, ew = L.affinity(raw=True)
-    oi, oj, ow = R.affinity_raw()
-    assert np.array_equal(ei, oi) and np.array_equal(ej, oj)
-    np.testing.assert_allclose(ew, ow, rtol=1e-5)
-    ei, ej, ew = L.affinity(raw=False)
-    oi, oj, ow = R.affinity()
-    assert np.array_equal(ei, oi) and np.array_equal(ej, oj)
-    np.testing.assert_allclose(ew, ow, rtol=1e-4, atol=1e-12)
-    assert L.stats()["lines3D"] == R.num_lines()
-    mr, rr = L.residuals(), R.residuals()
-    assert all(np.array_equal(mr[f], rr[f]) for f in ("line", "cam", "seg"))
-    ms, rs = L.segments3d(), R.segments3d()
-    assert np.array_equal(ms["line"], rs["line"])
-    a = np.sort(np.stack([ms["p1"], ms["p2"]], 1), axis=1)
-    b = np.sort(np.stack([rs["p1"], rs["p2"]], 1), axis=1)
-    np.testing.assert_allclose(a, b, rtol=0, atol=1e-6)      # TOLERANCE on 3D end points: 1e-6 scene units
-    return total, len(oi), R.num_lines()
+# weights: host libm vs libdevice; TOLERANCE on 3D end points: 1e-6 scene units
+STAGE_TOL = {"est_p_smp": dict(rtol=0, atol=1e-12), "affraw_w_smp": dict(rtol=1e-5), "aff_w_smp": dict(rtol=1e-4, atol=1e-12),
+             "seg_pts_smp": dict(rtol=0, atol=1e-6)}
 
 
 @pytest.mark.parametrize("diffusion,collin,knn", [(False, -1.0, 10), (True, -1.0, 10), (True, 2.0, 10), (False, -1.0, 0)])
-def test_synthetic_vs_reference_line3d_cc(ref_gpu, tmp_path, diffusion, collin, knn):
+def test_synthetic_vs_reference_line3d_cc(ref, diffusion, collin, knn):
     sc = synth.make_scene(12, 600, 41, "ring3", collinear=collin > 0)
     L = line3d.Line3D(neighbors_by_worldpoints=False, use_gpu=True)
     L.add_scene(sc)
     L.match_images(knn=knn)
     L.reconstruct_3d_lines(3, diffusion, collin)
-    R = ref_gpu.RefFullPipeline(False, True, "gpu", folder=str(tmp_path))
-    R.add_scene(sc)
-    R.match_images(knn=knn)
-    R.reconstruct(3, diffusion, collin)
-    total, nedges, nlines = compare_all_stages(L, R, sc.cam_ids, [len(s) for s in sc.segs], diffusion, collin)
-    assert total > 20000 and nedges > 3000 and nlines > 150, (total, nedges, nlines)
+    r = ref(f"full/{diffusion}_{collin}_{knn}")
+    util.check_record(util.product_record(L, sc.cam_ids, [len(s) for s in sc.segs], collin=collin > 0), r, STAGE_TOL)
+    assert r["scored_n"].sum() > 20000 and r["aff_n"] > 3000 and r["num_lines"] > 150, (r["scored_n"].sum(), r["aff_n"], r["num_lines"])
     L.close()
 
 
-def test_nvm_vs_reference_line3d_cc(ref_gpu, tmp_path):
+def test_nvm_vs_reference_line3d_cc(ref, tmp_path):
     """BASELINE configs[1]: testdata/vsfm_result.nvm (26 views, neighbours from world points, default parameters) through the
     product on the B200 and through the unmodified reference's CUDA path on the same GPU: matches_, estimated_position3D_, A_,
     local ids, clusters and 3D segments index-exact; and the two text result files agree value by value."""
@@ -96,24 +47,18 @@ def test_nvm_vs_reference_line3d_cc(ref_gpu, tmp_path):
     nu.add_all(L.add_image, inp)
     L.match_images()
     L.reconstruct_3d_lines(3, False)
-    R = ref_gpu.RefFullPipeline(True, True, "gpu", folder=str(tmp_path))
-    nu.add_all(R.add_view, inp)
-    R.match_images()
-    R.reconstruct(3, False)
-    total, nedges, nlines = compare_all_stages(L, R, range(inp["V"]), [len(s) for s in inp["segs"]], False, -1.0)
-    assert total > 1000000 and nlines > 2000, (total, nlines)
-    # result files: the reference's own writer vs the product's
-    name = R.save(str(tmp_path), txt=True)
-    (tmp_path / "mine").mkdir()
-    L.save_txt(str(tmp_path / "mine"))
-    ref_txt = open(tmp_path / (name + ".txt")).read().split()
-    my_txt = open(tmp_path / "mine" / (name + ".txt")).read().split()      # same file name (createOutputFilename)
-    assert len(ref_txt) == len(my_txt)
-    np.testing.assert_allclose(np.array(my_txt, float), np.array(ref_txt, float), rtol=1e-5, atol=1e-6)
+    nsegs = [len(s) for s in inp["segs"]]
+    r = ref("full/nvm")
+    mine = util.product_record(L, range(inp["V"]), nsegs)
+    # result files: the reference's own writer vs the product's, same file name (createOutputFilename)
+    L.save_txt(str(tmp_path))
+    v = np.array(open(tmp_path / (str(r["txt_name"]) + ".txt")).read().split(), float)
+    mine.update(txt_n=np.int64(len(v)), txt_smp=v[util.pick(len(v))], txt_name=r["txt_name"])
+    util.check_record(mine, r, dict(STAGE_TOL, txt_smp=dict(rtol=1e-5, atol=1e-6)))
+    assert r["scored_n"].sum() > 1000000 and r["num_lines"] > 2000, (r["scored_n"].sum(), r["num_lines"])
     # with diffusion on top (the reference supports re-running reconstruct3Dlines)
     L.reconstruct_3d_lines(3, True)
-    R.reconstruct(3, True)
-    compare_all_stages(L, R, range(inp["V"]), [len(s) for s in inp["segs"]], True, -1.0)
+    util.check_record(util.product_record(L, range(inp["V"]), nsegs), ref("full/nvm_diffusion"), STAGE_TOL)
     L.close()
 
 
@@ -125,7 +70,6 @@ def test_nvm_refcpu_semantics_vs_verbatim_cpu_reference_golden():
     matches, change the lists of later views: stated tolerance = at least 20 of 26 views with digest-identical scored lists,
     kept-match count within 0.5 %, line count within 1 %."""
     from tests import nvm_util as nu
-    from tests.test_ref_full_cpu import digest_matches, G
     inp = nu.load_inputs()
     z = np.load(os.path.join(G, "ref_full_nvm_cpu_v1.npz"))
     L = line3d.Line3D(neighbors_by_worldpoints=True, use_gpu=False)
